@@ -57,7 +57,15 @@ def parse_args():
                     help="which curve is the headline (value / ms_per_step); the other one is measured too and reported alongside")
     ap.add_argument("--strong-segments", type=int, default=64, help="segments of the fixed 100 M-row table of the strong-scaling curve")
     ap.add_argument("--no-variants", action="store_true", help="skip the 25 %% selectivity variant and the second scaling curve")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result table of the last timed headline step as DIR/<name>.npy (float64), so that two builds "
+                         "can be compared output for output on the same seeded table")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def measured_peak_gbs():
@@ -375,6 +383,24 @@ def parity_check(w, dist, threads):
     return {"groups": int(n), "docs_matched": int(docs), "ranks_checked": w.world}
 
 
+def result_arrays(table, q):
+    """The merged result table a caller of the hot path receives, copied out of the result's pinned memory as float64 arrays:
+    `keys` [groups, group-by columns], one array per aggregation named after it (COUNT from the long slot, SUM / MIN / MAX
+    from the double slot) and `stats` (docs scanned, entries scanned in / post filter, total docs).  A GROUP BY without
+    ORDER BY returns its groups in no defined order, so the rows are put in key order.  The bench query has at most
+    8 x 16 x 32 groups: well under a megabyte in all."""
+    from pinot_b200.query import AggOp
+    keys = np.stack([np.asarray(v, dtype=np.float64) for v in table.key_values], axis=1)
+    order = np.lexsort(keys.T[::-1])
+    out = {"keys": keys[order]}
+    for a, agg in enumerate(q.aggregations):
+        src = table.longs if agg.op == AggOp.COUNT else table.doubles
+        out[f"{agg.op.name.lower()}_{agg.column or 'star'}"] = np.asarray(src[a], dtype=np.float64)[order]
+    out["stats"] = np.array([table.stats[k] for k in ("num_docs_scanned", "num_entries_scanned_in_filter",
+                                                      "num_entries_scanned_post_filter", "num_total_docs")], dtype=np.float64)
+    return out
+
+
 def run_timed(w, steps, warmup, torch, dist, sampler=None):
     """W warm-up steps, then exactly K timed steps bracketed by barrier + synchronize; returns the timing record (max over
     ranks) and the per-kernel CUDA-event times measured by the library on the call's stream."""
@@ -466,6 +492,7 @@ def main():
     sampler.start()
     T = run_timed(w, args.steps, args.warmup, torch, dist, sampler)
     elapsed, last = T["elapsed"], T["last"]
+    outputs = result_arrays(last.tables[0], q) if args.dump_outputs else None
     # A K-step region of this workload lasts only a few ms, shorter than a handful of NVML reads: keep the SAME steps
     # running (untimed, same count on every rank) right after it so the clock median is taken under the identical load.
     n_extra = 0 if elapsed >= 0.25 else min(5000, int(0.25 / max(elapsed / max(args.steps, 1), 1e-5)))
@@ -654,6 +681,10 @@ def main():
                              "all": [round(float(x), 3) for x in T["step_wall"]]}, "host_us_by_phase": T["host_us"],
             "num_groups": int(num_groups), "docs_matched": int(docs_matched),
             "kernel_variant": {0: "tma+width-specialised", 4: "tma+generic", 8: "ldg+width-specialised", 12: "ldg+generic"}.get(args.flags & 12)}
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     _emit(line)
     if world > 1:
         _teardown(native, dist)

@@ -275,6 +275,7 @@ int pb_result_phase_ms(pb_result_handle r, double* filter_kernel_ms, double* agg
 int32_t pb_result_kernel_launches(pb_result_handle r);
 double pb_result_comm_ms(pb_result_handle r);           /* device time of the cross-rank merge (collective + merge kernel) */
 int32_t pb_result_in_place_columns(pb_result_handle r);   /* (segment, column) pairs this query gathered in place from host memory */
+int32_t pb_result_residual_leaves(pb_result_handle r);    /* (segment, filter leaf) pairs the aggregation kernel tested on its rows */
 /* host-side microseconds spent in this call, by phase: [0] resolve + stage, [1] table allocation + init,
  * [2] descriptor build + upload, [3] kernel launches, [4] wait for the scan + group count, [5] compaction,
  * gathers and read-back, [6] host key decode / stats; [7] reserved */

@@ -186,7 +186,8 @@ struct DevQuery {
   uint64_t n_units;
   uint64_t n_docs_total;
   int32_t match_all;                     // no filter: pb_agg_kernel walks every doc, no match list
-  int32_t pad_p;
+  int32_t agg_counts_docs;               // some segment has residual leaves (DevRowLeaf): the match list holds candidates and
+                                         // pb_agg_rows_kernel, not the filter kernel, counts docs_matched
   int32_t sparse_max;                    // survivors per 1024 docs below which later AND leaves use the restricted scan
   int32_t cand_bytes;                    // shared memory for the per-warp candidate lists (0: no leaf runs on candidates)
   uint64_t unit_lo;                      // this launch covers work units [unit_lo, unit_lo + n_units) (a wave of segments)
@@ -1246,7 +1247,7 @@ __global__ void __launch_bounds__(PB_NTHREADS, MIN_CTAS) pb_filter_kernel(const 
     }
     flush_out();
     // ---- segment exit: numDocsScanned of this segment's table (matched is warp-uniform) ----
-    if (lane == 0 && matched) pb_red_add_u64(Q.tables[sq.table].docs_matched, matched);
+    if (lane == 0 && matched && !Q.agg_counts_docs) pb_red_add_u64(Q.tables[sq.table].docs_matched, matched);
   }
 }
 
@@ -1509,19 +1510,40 @@ static __global__ void __launch_bounds__(PB_AGG_SMEM_THREADS, 1) pb_agg_smem_ker
 // per-column descriptors, no dictionary lookups, no bounds checks -- ~90 instructions per doc instead of the ~400 of the
 // general kernel, which was instruction- and latency-bound (ncu, profiles/r2_kernels.md).  RW = 32-bit words per row.
 // Table update: the CTA-private shared-memory table (SmemTable) when the launch carries one and has enough matches, else
-// reductions into the global table.
+// reductions into the global table.  Residual filter leaves (DevRowLeaf) are tested on the row before either.
 // ------------------------------------------------------------------------------------------------
 struct DevRowKey { uint32_t off, bits; uint64_t mult; const int32_t* remap; };
 struct DevRowAgg { uint32_t off, width, type, exact_int; };  // width 4 / 8 bytes, type PB_INT .. PB_DOUBLE; unused for COUNT(*).  exact_int: SUM / AVG
                                                              // of an integer column whose sums stay below 2^53 (same flag in every segment)
+// A RESIDUAL leaf: a dictionary leaf of a flat AND that would run on the filter kernel's candidates (DevLeaf::gather) and
+// whose column is a field of the row group.  The filter kernel leaves it out and hands its survivors over as candidates;
+// this kernel tests the leaf on the row it loads anyway, so a candidate's row is read once instead of twice.
+struct DevRowLeaf {
+  uint32_t off, bits;       // dictId field of the row
+  uint32_t lo, span;        // set == nullptr: match iff (dictId - lo) < span (unsigned)
+  const uint32_t* set;      // IN / NOT IN: bitset over dictIds, bit ^ excl
+  uint32_t excl, pad;
+};
+#define PB_ROWS_MAX_LEAVES 4
 struct DevRowSeg {
   const uint32_t* rows;
   uint64_t doc_base;
-  int32_t table, pad;
+  int32_t table, n_leaves;
   DevRowKey keys[PB_MAX_GROUP_BY];
   DevRowAgg aggs[PB_MAX_AGGS];
+  DevRowLeaf leaves[PB_ROWS_MAX_LEAVES];
 };
 #define PB_ROWS_SMEM_SEGS 16
+
+// field of `bits` bits at bit `off` of a row held in registers (words already byte-swapped, MSB first)
+template <int RW>
+__device__ __forceinline__ uint32_t pb_row_field(const uint32_t (&w)[RW], uint32_t off, uint32_t bits) {
+  const uint32_t wi = off >> 5, sh = off & 31u;
+  uint32_t hi = w[0], lo = RW > 1 ? w[1 % RW] : 0u;
+#pragma unroll
+  for (int k = 1; k < RW; k++) if (wi == (uint32_t)k) { hi = w[k]; lo = k + 1 < RW ? w[(k + 1) % RW] : 0u; }
+  return __funnelshift_l(lo, hi, sh) >> (32u - bits);
+}
 
 template <int RW>
 __global__ void __launch_bounds__(PB_AGG_SMEM_THREADS, 1) pb_agg_rows_kernel(const __grid_constant__ DevQuery Q, const DevRowSeg* __restrict__ gsegs) {
@@ -1572,13 +1594,7 @@ __global__ void __launch_bounds__(PB_AGG_SMEM_THREADS, 1) pb_agg_rows_kernel(con
   // the aggregation is latency-bound (ncu: 34 warps waiting on memory per issue slot when every field was its own load),
   // so the chain per doc is kept at match list -> row -> remap, and every thread works on two docs at a time.
   auto process = [&](unsigned long long gdoc, const uint32_t (&w)[RW], const DevRowSeg& sg) {
-    auto field = [&](uint32_t off, uint32_t bits) -> uint32_t {
-      const uint32_t wi = off >> 5, sh = off & 31u;
-      uint32_t hi = w[0], lo = RW > 1 ? w[1 % RW] : 0u;
-#pragma unroll
-      for (int k = 1; k < RW; k++) if (wi == (uint32_t)k) { hi = w[k]; lo = k + 1 < RW ? w[(k + 1) % RW] : 0u; }
-      return __funnelshift_l(lo, hi, sh) >> (32u - bits);
-    };
+    auto field = [&](uint32_t off, uint32_t bits) -> uint32_t { return pb_row_field<RW>(w, off, bits); };
     uint64_t slot = 0;
     for (int j = 0; j < nG; j++) {
       const DevRowKey& k = sg.keys[j];
@@ -1667,6 +1683,23 @@ __global__ void __launch_bounds__(PB_AGG_SMEM_THREADS, 1) pb_agg_rows_kernel(con
 #pragma unroll
     for (int k = 0; k < RW; k++) w[k] = pb_bswap32(w[k]);
   };
+  // the residual leaves of the doc's segment against its row: a candidate that fails one is dropped before any table update
+  auto passes = [&](const uint32_t (&w)[RW], const DevRowSeg& sg) -> bool {
+    for (int k = 0; k < sg.n_leaves; k++) {
+      const DevRowLeaf& l = sg.leaves[k];
+      const uint32_t id = pb_row_field<RW>(w, l.off, l.bits);
+      const bool ok = l.set ? (((__ldg(l.set + (id >> 5)) >> (id & 31)) & 1u) ^ l.excl) != 0u : (id - l.lo) < l.span;
+      if (!ok) return false;
+    }
+    return true;
+  };
+  // docs_matched (Q.agg_counts_docs): passing docs counted per thread for one table at a time
+  int cnt_table = 0;
+  uint32_t cnt = 0;
+  auto count = [&](int table) {
+    if (table != cnt_table && cnt) { pb_red_add_u64(Q.tables[cnt_table].docs_matched, cnt); cnt = 0; }
+    cnt_table = table; cnt++;
+  };
   const unsigned long long stride = (unsigned long long)gridDim.x * PB_AGG_SMEM_THREADS;
   for (unsigned long long i = (unsigned long long)blockIdx.x * PB_AGG_SMEM_THREADS + tid; i < n; i += 2 * stride) {
     const bool two = i + stride < n;
@@ -1677,8 +1710,22 @@ __global__ void __launch_bounds__(PB_AGG_SMEM_THREADS, 1) pb_agg_rows_kernel(con
     uint32_t w0[RW], w1[RW];
     load_row(sg0, gdoc0, w0);
     load_row(sg1, gdoc1, w1);
-    process(gdoc0, w0, sg0);
-    if (two) process(gdoc1, w1, sg1);
+    const bool ok0 = passes(w0, sg0), ok1 = two && passes(w1, sg1);
+    if (ok0) process(gdoc0, w0, sg0);
+    if (ok1) process(gdoc1, w1, sg1);
+    if (Q.agg_counts_docs) { if (ok0) count(sg0.table); if (ok1) count(sg1.table); }
+  }
+  if (Q.agg_counts_docs) {
+    // one reduction per warp when its lanes counted for one table (always so with PB_Q_COMBINE), else one per lane
+    const unsigned has = __ballot_sync(0xffffffffu, cnt != 0);
+    if (has) {
+      const int leader = __ffs(has) - 1;
+      const int t0 = __shfl_sync(0xffffffffu, cnt_table, leader);
+      if (__all_sync(0xffffffffu, cnt == 0 || cnt_table == t0)) {
+        const uint32_t sum = __reduce_add_sync(0xffffffffu, cnt);
+        if ((tid & 31) == leader) pb_red_add_u64(Q.tables[t0].docs_matched, sum);
+      } else if (cnt) pb_red_add_u64(Q.tables[cnt_table].docs_matched, cnt);
+    }
   }
   if (!use_smem) return;
   __syncthreads();

@@ -1015,6 +1015,7 @@ struct pb_result_s {
   std::vector<int> agg_filter_of;
   int waves = 1;                            // launches were split into this many waves behind the staging copies
   int in_place_columns = 0;                 // (segment, column) pairs gathered from mapped host memory (PB_Q_GATHER_IN_PLACE)
+  int residual_leaves = 0;                  // (segment, filter leaf) pairs tested by pb_agg_rows_kernel (DevRowLeaf)
   std::vector<int> agg_op;
   std::vector<std::string> gb_names, agg_cols;
   std::vector<TableMeta> tables;
@@ -2093,6 +2094,33 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
   size_t bm_off = 0;
   r->seg_scan_leaves.assign(n_segs, 0);
 
+  // ---- plan-time specialisation of the aggregation (pb_agg_rows_kernel): a dense table, every key a dictionary column
+  // and every aggregation COUNT(*) or a numeric column, all of them fields of row groups of one stride ----
+  int rows_rw = 0;
+  bool rows_ok = false;
+  {
+    static const bool rows_on = []() { const char* e = getenv("PB_AGG_ROWS"); return !e || atoi(e) != 0; }();
+    rows_ok = rows_on && table_mode == T_DENSE && nF == 0 && nG > 0 && n_segs > 0;
+    for (int si = 0; si < n_segs && rows_ok; si++) {
+      const RowGroup* rg = seg_rg[si];
+      if (!rg || (rows_rw && rows_rw != rg->stride_bits / 32)) { rows_ok = false; break; }
+      rows_rw = rg->stride_bits / 32;
+      for (int j = 0; j < nG && rows_ok; j++) if (rg->find(gcol[si][j], 0) < 0) rows_ok = false;
+      for (int a = 0; a < nA && rows_ok; a++) {
+        const int op = q->aggregations[a].op;
+        if (op == PB_AGG_COUNT) continue;
+        if (op == PB_AGG_DISTINCTCOUNT || rg->find(acol[si][a], 1) < 0) rows_ok = false;
+      }
+    }
+    if (!rows_ok) rows_rw = 0;
+  }
+  // Residual leaves (DevRowLeaf): with the rows kernel, a dictionary leaf that would run on the filter kernel's candidates
+  // and whose column is a row-group field leaves the filter program; the rows kernel tests it on the row it loads anyway.
+  // (PB_AGG_RESIDUAL=0 keeps such leaves on the candidates.)
+  static const bool residual_on = []() { const char* e = getenv("PB_AGG_RESIDUAL"); return !e || atoi(e) != 0; }();
+  std::vector<std::vector<DevRowLeaf>> residual(n_segs);
+  r->residual_leaves = 0;
+
   for (int si = 0; si < n_segs; si++) {
     pb_segment_s* s = g->segs[si];
     const pb_segment_query& sq = sqs[si];
@@ -2101,6 +2129,7 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
     ds.table = combine ? 0 : si;
     int n_scan = 0, set_smem_used = 0;
     int slot_of_col[PB_MAX_SCAN_SLOTS];
+    std::vector<char> residual_node((size_t)std::max(sq.num_filter_nodes, 0), 0);
     // one postfix filter program -> device nodes + leaves.  force_gather: every scan leaf is tested per doc from its forward
     // index (FILTER clauses, evaluated by pb_agg_kernel); otherwise the candidate plan decides per leaf.
     auto build_program = [&](const pb_filter_node* nodes, int n_nodes, int8_t* node_kind, int8_t* node_arg, DevLeaf* leaves, int max_leaves,
@@ -2118,6 +2147,16 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
       lf.set_smem_off = -1;
       lf.est_permille = 500;
       node_kind[n] = N_LEAF; node_arg[n] = (int8_t)n_leaves; n_leaves++;
+      // row-group field of a residual leaf, -1 = the leaf stays in this program
+      const int residual_field = (!force_gather && rows_ok && residual_on && cand_leaf[si][n] && residual[si].size() < PB_ROWS_MAX_LEAVES &&
+                                  (fn.kind == PB_F_SCAN_DICT_RANGE || fn.kind == PB_F_SCAN_DICT_SET)) ? seg_rg[si]->find(fn.column, 0) : -1;
+      auto make_residual = [&](const Column& c, const uint32_t* set) {
+        DevRowLeaf rl; memset(&rl, 0, sizeof rl);
+        rl.off = (uint32_t)seg_rg[si]->bit_off[(size_t)residual_field]; rl.bits = (uint32_t)c.bits;
+        rl.lo = lf.lo; rl.span = lf.span; rl.set = set; rl.excl = (uint32_t)lf.exclusive;
+        residual[si].push_back(rl);
+        residual_node[n] = 1;
+      };
       auto scan_slot = [&](const Column& c) -> int {
         if (force_gather || cand_leaf[si][n]) {          // evaluated on candidates: no stage slot, read where the column lies
           lf.gather = 1;
@@ -2154,7 +2193,8 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
           if (lo == 0 && hi >= c.card) { lf.kind = L_TRUE; break; }
           lf.kind = L_DICT_RANGE; lf.bits = c.bits; lf.lo = (uint32_t)lo; lf.span = (uint32_t)(hi - lo);
           lf.est_permille = (int32_t)(1000.0 * (double)(hi - lo) / (double)c.card);
-          if ((lf.slot = scan_slot(c)) < 0) return fail(PB_ERR_UNSUPPORTED, "more than %d scanned columns", PB_MAX_SCAN_SLOTS);
+          if (residual_field >= 0) make_residual(c, nullptr);
+          else if ((lf.slot = scan_slot(c)) < 0) return fail(PB_ERR_UNSUPPORTED, "more than %d scanned columns", PB_MAX_SCAN_SLOTS);
           r->seg_scan_leaves[si]++;
           break;
         }
@@ -2173,8 +2213,11 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
           lf.kind = L_DICT_SET; lf.bits = c.bits; lf.exclusive = fn.exclusive ? 1 : 0;
           lf.set_bits = dbits; lf.set_card = c.card;
           { double f = (double)fn.num_ids / (double)c.card; lf.est_permille = (int32_t)(1000.0 * (fn.exclusive ? 1.0 - f : f)); }
-          if (!force_gather && set_smem_used + c.card <= PB_SET_SMEM_BYTES) { lf.set_smem_off = set_smem_used; set_smem_used += (c.card + 15) & ~15; }
-          if ((lf.slot = scan_slot(c)) < 0) return fail(PB_ERR_UNSUPPORTED, "more than %d scanned columns", PB_MAX_SCAN_SLOTS);
+          if (residual_field >= 0) make_residual(c, dbits);
+          else {
+            if (!force_gather && set_smem_used + c.card <= PB_SET_SMEM_BYTES) { lf.set_smem_off = set_smem_used; set_smem_used += (c.card + 15) & ~15; }
+            if ((lf.slot = scan_slot(c)) < 0) return fail(PB_ERR_UNSUPPORTED, "more than %d scanned columns", PB_MAX_SCAN_SLOTS);
+          }
           r->seg_scan_leaves[si]++;
           break;
         }
@@ -2248,6 +2291,21 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
     {
       int nl = 0;
       if ((rc = build_program(sq.filter, sq.num_filter_nodes, ds.node_kind, ds.node_arg, ds.leaves, PB_MAX_LEAVES, nl, false))) return rc;
+      if (!residual[si].empty()) {
+        // the program is a flat AND (candidate leaves exist only there) whose leaf i is node i: keep the other leaves, which
+        // include the streamed one, under an AND of their number
+        int kept = 0;
+        for (int n = 0; n + 1 < sq.num_filter_nodes; n++) {
+          if (residual_node[n]) continue;
+          ds.leaves[kept] = ds.leaves[ds.node_arg[n]];
+          ds.node_kind[kept] = N_LEAF; ds.node_arg[kept] = (int8_t)kept;
+          kept++;
+        }
+        ds.node_kind[kept] = N_AND; ds.node_arg[kept] = (int8_t)kept;
+        ds.n_nodes = kept + 1;
+        for (int l = kept; l < nl; l++) memset(&ds.leaves[l], 0, sizeof(DevLeaf));
+        r->residual_leaves += (int)residual[si].size();
+      }
     }
     // FILTER(WHERE ...) clauses
     ds.n_agg_filters = nF;
@@ -2311,25 +2369,10 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
     }
   }
 
-  // ---- plan-time specialisation of the aggregation (pb_agg_rows_kernel): a dense table, every key a dictionary column
-  // and every aggregation COUNT(*) or a numeric column, all of them fields of row groups of one stride ----
+  // ---- the rows kernel's per-segment descriptors ----
   const DevRowSeg* d_row_segs = nullptr;
-  int rows_rw = 0;
-  {
-    static const bool rows_on = []() { const char* e = getenv("PB_AGG_ROWS"); return !e || atoi(e) != 0; }();
-    bool ok = rows_on && table_mode == T_DENSE && nF == 0 && nG > 0 && n_segs > 0;
-    for (int si = 0; si < n_segs && ok; si++) {
-      const RowGroup* rg = seg_rg[si];
-      if (!rg || (rows_rw && rows_rw != rg->stride_bits / 32)) { ok = false; break; }
-      rows_rw = rg->stride_bits / 32;
-      for (int j = 0; j < nG && ok; j++) if (rg->find(gcol[si][j], 0) < 0) ok = false;
-      for (int a = 0; a < nA && ok; a++) {
-        const int op = q->aggregations[a].op;
-        if (op == PB_AGG_COUNT) continue;
-        if (op == PB_AGG_DISTINCTCOUNT || rg->find(acol[si][a], 1) < 0) ok = false;
-      }
-    }
-    if (ok) {
+  if (rows_ok) {
+    {
       DevRowSeg* h_rs = nullptr;
       d_row_segs = ar.put<DevRowSeg>(nullptr, (size_t)n_segs, &h_rs);
       if (!d_row_segs) return fail(PB_ERR_STATE, "query arena overflow");
@@ -2351,6 +2394,8 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
           rs.aggs[a].off = (uint32_t)rg->bit_off[(size_t)rg->find(acol[si][a], 1)];
           rs.aggs[a].width = (uint32_t)c.entry_bytes; rs.aggs[a].type = (uint32_t)c.type; rs.aggs[a].exact_int = 0;
         }
+        rs.n_leaves = (int32_t)residual[si].size();
+        for (int k = 0; k < rs.n_leaves; k++) rs.leaves[k] = residual[si][(size_t)k];
       }
       // SUM / AVG over INT / LONG columns: when max|value| x docs < 2^53 every partial sum is an integer a double holds
       // exactly, so the CTA-private table may accumulate them as 64-bit integers with two native 32-bit shared-memory
@@ -2376,7 +2421,7 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
         }
         if (exact) for (int si = 0; si < n_segs; si++) h_rs[si].aggs[a].exact_int = 1;
       }
-    } else rows_rw = 0;
+    }
   }
 
   // ---- work-unit geometry: one stage = one unit (U x 1024 docs) of every scan slot, per warp ----
@@ -2517,6 +2562,7 @@ static int exec_single(pb_segment_group_handle g, const pb_segment_query* sqs, c
   hq->generic = (q->flags & PB_Q_GENERIC_KERNEL) ? 1 : 0;
   hq->n_units = n_chunks; hq->segs = dsegs; hq->tables = dtabs;
   hq->n_docs_total = n_docs_total; hq->match_all = match_all ? 1 : 0;
+  hq->agg_counts_docs = r->residual_leaves > 0 ? 1 : 0;
   { static const int sm = []() { const char* e = getenv("PB_SPARSE_MAX"); return e ? atoi(e) : PB_SPARSE_MAX; }(); hq->sparse_max = sm; }
   hq->match_list = d_match_list;
   if (use_smem_table) {
@@ -3302,6 +3348,7 @@ extern "C" int pb_result_wait(pb_result_handle r) {
   return PB_OK;
 }
 extern "C" int32_t pb_result_in_place_columns(pb_result_handle r) { return r ? r->in_place_columns : 0; }
+extern "C" int32_t pb_result_residual_leaves(pb_result_handle r) { return r ? r->residual_leaves : 0; }
 extern "C" double pb_result_comm_ms(pb_result_handle r) {
   if (!r || !r->comm_timed) return 0;
   if (r->comm_ms == 0) { float ms = 0; cudaEventSynchronize(r->sset.ev[6]); if (cudaEventElapsedTime(&ms, r->sset.ev[5], r->sset.ev[6]) == cudaSuccess) r->comm_ms = ms; }

@@ -151,6 +151,8 @@ def lib():
     l.pb_result_kernel_launches.restype = C.c_int32
     l.pb_result_in_place_columns.argtypes = [C.c_void_p]
     l.pb_result_in_place_columns.restype = C.c_int32
+    l.pb_result_residual_leaves.argtypes = [C.c_void_p]
+    l.pb_result_residual_leaves.restype = C.c_int32
     l.pb_result_stream.argtypes = [C.c_void_p]
     l.pb_result_stream.restype = C.c_void_p
     l.pb_result_wait.argtypes = [C.c_void_p]
@@ -407,6 +409,7 @@ class Result:
         self.query = q
         self._finalized = not deferred
         self.in_place_columns = lib().pb_result_in_place_columns(rh)     # known as soon as the call is planned
+        self.residual_leaves = lib().pb_result_residual_leaves(rh)       # filter leaves tested by the aggregation kernel
         if not deferred:
             self._load()
 
